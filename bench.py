@@ -5,6 +5,7 @@ rank takes 32 pages of the round-robin shard, i.e. configs[2] at 8 GPUs; weak sc
 
   python bench.py --gpus N --steps K --warmup W                      # ours (hand-written CUDA through the C ABI)
   python bench.py --impl reference --gpus N --steps K --warmup W     # CPU restatement of the reference path (oracle/)
+  python bench.py ... --dump-outputs DIR                              # also write the last timed step's results as DIR/*.npy
 
 One JSON line on stdout (rank 0).  `value` = device-resident throughput (inputs staged in HBM, CUDA-event timed, max over
 ranks); `e2e` = the same pages through the plugin `infer` calls with pinned HOST buffers (H2D/D2H and host glue inside
@@ -18,6 +19,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -33,6 +35,13 @@ PAGE_H, PAGE_W, LINES = 2048, 1536, 32
 PAGES_PER_GPU = 32
 VOCAB = 46000
 METRIC = "pages/sec (2048x1536, detect+OCR+inpaint)"
+DUMP_PAGES = 32                                   # --dump-outputs: the first 32 pages of the step (all of them by default)
+DUMP_SAMPLES = {"db": 65536, "db_mask": 32768, "inpainted": 131072}     # sampled elements per page: 28 MB at 32 pages
+
+# The plugins get their weights in memory, but constructing one creates its model directory (default ./models).  Point it at a
+# temporary directory so that the benchmark writes nothing into the tree it runs from, which may be read-only.
+_MODEL_DIR = tempfile.TemporaryDirectory(prefix="mitb_models_")
+os.environ.setdefault("MITB_MODEL_DIR", _MODEL_DIR.name)
 
 
 def log(*a):
@@ -409,6 +418,38 @@ def c4_figure(hp, n_pages):
             "uint8 in / uint8 out incl. pack, blend and composite; bottleneck 320x240x512, FFT 320x240"}
 
 
+def dump_outputs(results, out_dir):
+    """Writes what `HotPath.run_resident` returned for each page of one step, as float32 arrays indexed [page, ...]:
+    db / db_mask / inpainted are a fixed seeded sample of elements (the same positions on every page) of the detector's
+    probability map [1,2,H,W], its mask [1,1,H/2,W/2] and the inpainted uint8 page [H,W,3]; ocr_* hold every text line in
+    chunk order (lines sorted by width, as run_resident feeds them) with the collapsed CTC results compacted to the front
+    and zero past ocr_counts.  Total size at most ~40 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    results = results[:DUMP_PAGES]
+    arrays = {}
+    for seed, (name, pick) in enumerate((("db", lambda r: r[0]), ("db_mask", lambda r: r[1]), ("inpainted", lambda r: r[3]))):
+        n = pick(results[0]).numel()
+        idx = np.sort(np.random.default_rng(seed).choice(n, size=min(DUMP_SAMPLES[name], n), replace=False))
+        idx = torch.from_numpy(idx).to(pick(results[0]).device)
+        arrays[name] = torch.stack([pick(r).reshape(-1)[idx].float() for r in results]).cpu().numpy()
+    lines = [[(c, t) for c in [[x.cpu() for x in chunk] for chunk in r[2]] for t in range(c[0].shape[0])] for r in results]   # (chunk, row) per line
+    n_lines = max(len(l) for l in lines)
+    T = max(c[1].shape[1] for r in results for c in r[2])
+    counts = np.zeros((len(results), n_lines), np.float32)
+    steps, chars, logprob = (np.zeros((len(results), n_lines, T), np.float32) for _ in range(3))
+    colors = np.zeros((len(results), n_lines, T, 6), np.float32)
+    for p, page_lines in enumerate(lines):
+        for i, (c, t) in enumerate(page_lines):
+            k = int(c[0][t])
+            counts[p, i] = k
+            for dst, src in ((steps, c[1]), (chars, c[2]), (logprob, c[3]), (colors, c[4])):
+                dst[p, i, :k] = src[t, :k].float().numpy()
+    arrays.update(ocr_counts=counts, ocr_steps=steps, ocr_chars=chars, ocr_logprob=logprob, ocr_colors=colors)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    log(f"[bench] wrote {len(arrays)} arrays ({sum(a.nbytes for a in arrays.values()) / 1e6:.1f} MB) of the last timed step to {out_dir}")
+
+
 def run_ours(args, rank, world, local_rank):
     import torch.distributed as dist
     from mit_b200 import exchange, synth
@@ -452,19 +493,25 @@ def run_ours(args, rank, world, local_rank):
     # multi-GPU: fixed-size result records (boxes, scores, OCR text / colours, raw mask, inpainted page) all-gathered over NCCL
     xchg = ResultExchange(dev, len(pages), PAGE_H, PAGE_W) if world > 1 else None
 
-    def resident_step():
+    def resident_step(keep=False):
+        kept = []
         for i, sp in enumerate(staged):
             db, dmask, ocr, out = hp.run_resident(sp)
+            if keep:                                         # --dump-outputs: hold this step's results (fresh tensors per call)
+                kept.append((db, dmask, ocr, out))
             if xchg is not None:                             # N > 1: the page goes into this rank's result record, device to device
                 o, nb = xchg.lay.o["page"]
                 xchg.buf[i, o:o + nb].copy_(out.reshape(-1))
         if xchg is not None:
             exchange.gather_records(xchg.buf, world)         # the one collective of the path: all ranks' records over NCCL / NVLink
-        return out
+        return kept
 
     # ---------------- device-resident throughput (`value`)
+    # --dump-outputs holds the last timed step's results; the warm-up steps hold theirs too, so that the allocator has that memory
+    # cached before the timed region instead of allocating it inside
+    dump = args.dump_outputs is not None and rank == 0
     for _ in range(args.warmup):
-        resident_step()
+        resident_step(keep=dump)
     barrier()
     eng.lib.mitb_profile_enable(eng._h, 1)
     clocks = ClockSampler(local_rank)
@@ -473,8 +520,8 @@ def run_ours(args, rank, world, local_rank):
     launches0 = eng.launches
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(args.steps):
-        resident_step()
+    for step in range(args.steps):
+        last = resident_step(keep=dump and step == args.steps - 1)
     e1.record()
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
@@ -491,6 +538,9 @@ def run_ours(args, rank, world, local_rank):
     e1.record()
     barrier()
     value_unprofiled = n_pages * world / (max_over_ranks(e0.elapsed_time(e1)) / 1e3)
+    if dump:
+        dump_outputs(last, args.dump_outputs)
+    del last
 
     # ---------------- end-to-end through the plugin API with host buffers (`e2e`)
     def e2e_step():
@@ -603,7 +653,7 @@ def run_ours(args, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3, help="timed steps (each runs every page once)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "reference-cuda"])
     ap.add_argument("--pages", type=int, default=PAGES_PER_GPU, help="pages per GPU per step (BASELINE configs[1]: 32)")
@@ -613,7 +663,11 @@ def main():
     ap.add_argument("--no-c4", action="store_true", help="skip the lama_large @ 2560 (BASELINE configs[3]) figure")
     ap.add_argument("--workers", type=int, default=8, help="host threads of the page pipeline in the e2e leg")
     ap.add_argument("--fast-e2e", action="store_true", help="one warm-up step for the e2e leg (development only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                                                          "(float32; inputs are seeded, so runs with the same arguments compare output for output)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0 or args.pages < 1:
+        ap.error("--steps and --pages must be >= 1, --warmup >= 0")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":

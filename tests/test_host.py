@@ -1,10 +1,10 @@
 """Host-side logic (no GPU): geometry / detector post-processing / MPE tables / CTC collapse / rearrangement / the C ABI
-surface.  Where the reference helper is importable here (build container) it is the checker; otherwise the oracle is."""
+surface.  Where a reference helper is the checker, its outputs on seeded inputs are stored under tests/golden."""
 import asyncio
 import ctypes
+import json
 import os
 import re
-import warnings
 
 import cv2
 import numpy as np
@@ -12,10 +12,9 @@ import pytest
 
 from mit_b200 import synth
 from mit_b200.host import det_post, geometry, mpe, rearrange
-from oracle import nets, refload
+from oracle import cases, nets
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-needs_ref = pytest.mark.skipif(not refload.available(), reason="/root/reference not present")
 
 
 def test_abi_header_and_library_agree():
@@ -133,109 +132,65 @@ def test_synthetic_page_is_deterministic():
     assert [x.direction for x in q] == ["h"] * 3 + ["v"] * 3
 
 
-@needs_ref
+def _reference(name):
+    """What the reference helpers returned on the seeded inputs of oracle/cases.py (tests/golden, oracle/make_reference_golden.py)."""
+    path = os.path.join(ROOT, "tests", "golden", name)
+    if name.endswith(".json"):
+        with open(path) as f:
+            return json.load(f)
+    return np.load(path)
+
+
 def test_quadrilateral_matches_reference():
-    warnings.filterwarnings("ignore")
-    U = refload.load()["utils"]
-    rng = np.random.default_rng(4)
-    page, boxes, _ = synth.make_page(1, 1024, 768, 10)
-    for b in boxes + [np.array([[100, 100], [400, 130], [390, 190], [95, 160]]), np.array([[50, 50], [90, 60], [70, 400], [30, 390]])]:
-        b = b[rng.permutation(4)]
-        mine, ref = geometry.Quadrilateral(b, "", 1.0), U.Quadrilateral(b, "", 1.0)
-        assert np.array_equal(mine.pts, ref.pts) and mine.direction == ref.direction
-        assert abs(mine.aspect_ratio - ref.aspect_ratio) < 1e-6 and abs(mine.font_size - ref.font_size) < 1e-6
-        assert tuple(mine.aabb) == (ref.aabb.x, ref.aabb.y, ref.aabb.w, ref.aabb.h)
-        assert mine.is_approximate_axis_aligned == ref.is_approximate_axis_aligned and abs(mine.angle - ref.angle) < 1e-6
+    page, boxes = cases.quad_boxes()
+    want = _reference("ref_host.json")["quadrilateral"]
+    assert len(want) == len(boxes)
+    for b, ref in zip(boxes, want):
+        mine = geometry.Quadrilateral(b, "", 1.0)
+        assert mine.pts.tolist() == ref["pts"] and mine.direction == ref["direction"]
+        assert abs(mine.aspect_ratio - ref["aspect_ratio"]) < 1e-6 and abs(mine.font_size - ref["font_size"]) < 1e-6
+        assert list(mine.aabb) == ref["aabb"]
+        assert mine.is_approximate_axis_aligned == ref["axis_aligned"] and abs(mine.angle - ref["angle"]) < 1e-6
         for d in ("h", "v"):
-            assert np.array_equal(mine.get_transformed_region(page, d, 48), ref.get_transformed_region(page, d, 48))
+            assert cases.digest(mine.get_transformed_region(page, d, 48)) == ref["region"][d]
 
 
-@needs_ref
 def test_rearrange_matches_reference():
-    warnings.filterwarnings("ignore")
-    U = refload.load()["utils"]
-
-    def fwd(batch, device=None):
-        batch = np.asarray(batch).astype(np.float32)
-        s = batch.shape[1]
-        db = np.stack([batch[..., 0] / 255.0, batch[..., 1] / 255.0], 1).astype(np.float32)
-        mask = np.stack([cv2.resize(b[..., 2], (s // 2, s // 2)) / 255.0 for b in batch])[:, None].astype(np.float32)
-        return db, mask
-    rng = np.random.default_rng(0)
-    for shape in ((3000, 500, 3), (500, 3300, 3), (1024, 768, 3)):
-        img = cv2.GaussianBlur(rng.integers(0, 256, shape, dtype=np.uint8), (0, 0), 5)
-        r = U.det_rearrange_forward(img, fwd, 1024, 4)
-        o = rearrange.rearrange_forward(img, fwd, 1024, 4)
-        if r[0] is None:
+    want = _reference("ref_host.json")["rearrange"]
+    for img, r in zip(cases.rearrange_images(), want):
+        o = rearrange.rearrange_forward(img, cases.rearrange_forward_stub, 1024, 4)
+        if r is None:
             assert o[0] is None
         else:
-            assert np.array_equal(r[0], o[0]) and np.array_equal(r[1], o[1])
+            assert r == [cases.digest(o[0]), cases.digest(o[1])]
 
 
-@needs_ref
 def test_detector_helpers_match_reference():
-    warnings.filterwarnings("ignore")
-    refload.load()
-    import importlib
-    du = importlib.import_module("manga_translator.detection.default_utils.dbnet_utils")
-    ip = importlib.import_module("manga_translator.detection.default_utils.imgproc")
-    rep = du.SegDetectorRepresenter(0.5, 0.7, unclip_ratio=2.3)
-    rng = np.random.default_rng(5)
-    prob = cv2.GaussianBlur(rng.random((120, 160)).astype(np.float32), (0, 0), 4)
-    cnts, _ = cv2.findContours(((prob > prob.mean()) * 255).astype(np.uint8), cv2.RETR_LIST, cv2.CHAIN_APPROX_SIMPLE)
-    for c in cnts[:10]:
-        c = c.squeeze(1)
-        if len(c) < 3:
-            continue
-        a, b = det_post.mini_box(c), rep.get_mini_boxes(c)
-        assert np.allclose(np.array(a[0]), np.array(b[0])) and a[1] == b[1]
-        assert abs(det_post.box_score(prob, c) - rep.box_score_fast(prob, c)) < 1e-12
-    img = rng.integers(0, 256, (300, 200, 3), dtype=np.uint8)
+    want = _reference("ref_host.json")
+    prob, cnts, img = cases.contour_case()
+    assert len(cnts) == len(want["mini_boxes"])
+    for c, b in zip(cnts, want["mini_boxes"]):
+        a = det_post.mini_box(c)
+        assert np.allclose(np.array(a[0]), np.array(b["pts"])) and a[1] == b["sside"]
+        assert abs(det_post.box_score(prob, c) - b["score"]) < 1e-12
     for size in (512, 256, 300):
-        a, b = det_post.resize_aspect_ratio(img, size, cv2.INTER_LINEAR), ip.resize_aspect_ratio(img, size, cv2.INTER_LINEAR, mag_ratio=1)
-        assert np.array_equal(a[0], b[0]) and a[1:] == b[1:]
+        a, b = det_post.resize_aspect_ratio(img, size, cv2.INTER_LINEAR), want["resize_aspect_ratio"][str(size)]
+        assert cases.digest(a[0]) == b["image"] and cases.plain(a[1:]) == b["rest"]
 
 
-@needs_ref
 def test_boxes_from_prob_equals_reference_representer():
-    """D9 end to end: the reference's own SegDetectorRepresenter.boxes_from_bitmap (dbnet_utils.py:96-144) executed here, with the
-    two absent third-party calls adapted (pyclipper.PyclipperOffset -> our Clipper 6.4.2 restatement, shapely Polygon.area/.length ->
-    shoelace / perimeter), against host.det_post.boxes_from_prob: contour order, mini boxes, scores, thresholds, unclip call,
-    scale / clip / round / roll must agree EXACTLY (boxes int64 and scores)."""
-    warnings.filterwarnings("ignore")
-    refload.load()
-    import importlib
-    du = importlib.import_module("manga_translator.detection.default_utils.dbnet_utils")
-
-    class _Offset:
-        def AddPath(self, box, jt, et):
-            self.box = box
-
-        def Execute(self, d):
-            return [det_post.clipper_offset_round(self.box, d)]
-
-    class _Poly:
-        def __init__(self, b):
-            self.area, self.length = geometry.polygon_area(np.asarray(b, np.float64)), geometry.polygon_perimeter(np.asarray(b, np.float64))
-    saved = (du.pyclipper, du.Polygon)
-    du.pyclipper = type("pc", (), dict(PyclipperOffset=_Offset, JT_ROUND=1, ET_CLOSEDPOLYGON=2))
-    du.Polygon = _Poly
-    try:
-        rng = np.random.default_rng(11)
-        prob = (0.05 * rng.random((400, 600))).astype(np.float32)
-        for k in range(14):                                        # rotated / thin / tiny blobs, some below box_thresh
-            cx, cy, w, h, ang = rng.integers(40, 560), rng.integers(40, 360), rng.integers(3, 120), rng.integers(3, 40), rng.uniform(0, 180)
-            pts = cv2.boxPoints(((float(cx), float(cy)), (float(w), float(h)), float(ang))).astype(np.int32)
-            cv2.fillPoly(prob, [pts], float(rng.uniform(0.55, 0.99)))
-        rep = du.SegDetectorRepresenter(0.5, 0.7, unclip_ratio=2.3)
-        for (dw, dh) in ((600, 400), (1500, 1000)):
-            rb, rs = rep.boxes_from_bitmap(prob, prob > 0.5, dw, dh)
-            mb, ms = det_post.boxes_from_prob(prob, 0.5, 0.7, 2.3, dw, dh)
-            assert rb.shape == mb.shape and len(rb) >= 8
-            assert np.array_equal(rb, mb) and np.array_equal(rs, ms)
-            assert (mb.reshape(len(mb), -1).sum(1) > 0).sum() >= 3
-    finally:
-        du.pyclipper, du.Polygon = saved
+    """D9 end to end: the reference's own SegDetectorRepresenter.boxes_from_bitmap (dbnet_utils.py:96-144), run with the two absent
+    third-party calls adapted (pyclipper.PyclipperOffset -> our Clipper 6.4.2 restatement, shapely Polygon.area/.length -> shoelace /
+    perimeter), against host.det_post.boxes_from_prob: contour order, mini boxes, scores, thresholds, unclip call, scale / clip / round /
+    roll must agree EXACTLY (boxes int64 and scores)."""
+    g = _reference("ref_boxes_from_bitmap.npz")
+    prob = cases.blob_prob_map()                               # rotated / thin / tiny blobs, some below box_thresh
+    for (dw, dh) in ((600, 400), (1500, 1000)):
+        rb, rs = g[f"boxes_{dw}x{dh}"], g[f"scores_{dw}x{dh}"]
+        mb, ms = det_post.boxes_from_prob(prob, 0.5, 0.7, 2.3, dw, dh)
+        assert rb.shape == mb.shape and len(rb) >= 8
+        assert np.array_equal(rb, mb) and np.array_equal(rs, ms)
+        assert (mb.reshape(len(mb), -1).sum(1) > 0).sum() >= 3
 
 
 def test_bench_roofline_object_from_profile():

@@ -1,21 +1,15 @@
 """CPU tests of the mask-refinement row (SURVEY 8f N1): the oracle restatement (oracle/mask_refine_ref.py) against closed-form
 properties and hand-derived geometry, and the product's host logic (mit_b200/mask_refinement.py) against the oracle.
-pydensecrf and shapely are absent here and in /root/reference, so the DenseCRF part is `parity unpinned` (see the oracle's header)."""
+pydensecrf and shapely are not installed and not part of the reference tree, so the DenseCRF part is `parity unpinned` (see the oracle's header)."""
 import math
 import os
-import sys
-import types
 
 import cv2
 import numpy as np
-import pytest
 
-from mit_b200 import synth
 from mit_b200.host import geometry
+from oracle import cases
 from oracle import mask_refine_ref as R
-from oracle import refload
-
-needs_ref = pytest.mark.skipif(not refload.available(), reason="/root/reference not present")
 
 
 def _host_module():
@@ -82,14 +76,8 @@ def test_dense_crf_restatement_behaviour():
     assert (out != truth).mean() < 0.01 < (noisy != truth).mean()
 
 
-def _regions(boxes, k=2):
-    return [types.SimpleNamespace(lines=[b.astype(np.float64) for b in boxes[i:i + k]]) for i in range(0, len(boxes), k)]
-
-
-def _page(seed=3, h=768, w=576, n=8):
-    page, boxes, _ = synth.make_page(seed, h, w, n)
-    raw = cv2.dilate(((page[..., 0] < 100) * 255).astype(np.uint8), np.ones((3, 3), np.uint8))
-    return page, boxes, raw
+_regions = cases.refine_regions
+_page = cases.refine_page
 
 
 def test_assignment_product_equals_oracle():
@@ -124,97 +112,28 @@ def test_oracle_dispatch_on_synthetic_page():
     assert (out[box_area == 0] == 0).all()                        # ... and nothing far from the text lines is
 
 
-@needs_ref
+def _reference():
+    """What the reference's own code returned on these inputs (tests/golden, oracle/make_reference_golden.py)."""
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_mask_refinement.npz"))
+
+
 def test_scaled_float_lines_match_reference_quadrilateral():
     """dispatch builds Quadrilateral(line * scale_factor): float corners.  Our class must read them as the reference's does."""
-    U = refload.load()["utils"]
+    g = _reference()
     _, boxes, _ = _page()
-    for b in boxes + [np.array([[10, 20], [200, 35], [195, 80], [5, 66]])]:
-        a, r = R._Line(geometry.Quadrilateral, b * (2.0 / 3.0)), R._Line(U.Quadrilateral, b * (2.0 / 3.0))
-        assert np.array_equal(a.pts, r.pts) and a.font_size == r.font_size and np.array_equal(a.aabb_xywh, r.aabb_xywh)
+    for i, b in enumerate(boxes + [np.array([[10, 20], [200, 35], [195, 80], [5, 66]])]):
+        a = R._Line(geometry.Quadrilateral, b * (2.0 / 3.0))
+        assert np.array_equal(a.pts, g[f"line{i}_pts"]) and a.font_size == g[f"line{i}_font_size"] and np.array_equal(a.aabb_xywh, g[f"line{i}_aabb"])
 
 
-def _load_reference_mask_refinement():
-    """The reference's OWN mask_refinement package (`__init__.py` + `text_mask_utils.py`, unmodified) with its two absent third-party
-    dependencies bound to the oracle's restatements: shapely.geometry.Polygon (area / intersection / distance / centroid) and
-    pydensecrf (DenseCRF2D, unary_from_softmax)."""
-    import importlib
-    import importlib.util
-    refload.load()
-
-    class _Pt:
-        def __init__(self, x, y):
-            self.x, self.y = x, y
-
-    class Polygon:
-        def __init__(self, pts):
-            self.p = np.asarray(pts, dtype=np.float64).reshape(-1, 2)
-
-        @property
-        def area(self):
-            return R.poly_area(self.p) if len(self.p) >= 3 else 0.0
-
-        @property
-        def centroid(self):                                     # only ever asked of the component rectangle
-            return _Pt(float(self.p[:, 0].mean()), float(self.p[:, 1].mean()))
-
-        def intersection(self, other):                          # `other` is the axis-aligned component rectangle
-            x0, y0, x1, y1 = other.p[:, 0].min(), other.p[:, 1].min(), other.p[:, 0].max(), other.p[:, 1].max()
-            return Polygon(np.asarray(R.clip_poly_rect(self.p, x0, y0, x1, y1)).reshape(-1, 2))
-
-        def distance(self, pt):
-            return R.point_poly_distance(self.p, pt.x, pt.y)
-
-    class DenseCRF2D:
-        def __init__(self, w, h, n):
-            self.w, self.h, self.n = w, h, n
-
-        def setUnaryEnergy(self, u):
-            self.u = np.asarray(u, dtype=np.float32)
-
-        def addPairwiseGaussian(self, sxy, compat, kernel=None, normalization=None):
-            self.g = (float(sxy), float(compat))
-
-        def addPairwiseBilateral(self, sxy, srgb, rgbim, compat, kernel=None, normalization=None):
-            self.b, self.rgb = (float(sxy), float(srgb), float(compat)), np.asarray(rgbim)
-
-        def inference(self, n):
-            assert self.rgb.shape[:2] == (self.h, self.w)
-            return R.dense_crf_2d(self.rgb, self.u, n, self.g[0], self.g[1], self.b[0], self.b[1], self.b[2])
-
-    geom = sys.modules["shapely.geometry"]
-    geom.Polygon = Polygon
-    dcrf = types.ModuleType("pydensecrf.densecrf")
-    dcrf.DenseCRF2D, dcrf.DIAG_KERNEL, dcrf.NO_NORMALIZATION = DenseCRF2D, 1, 0
-    putils = types.ModuleType("pydensecrf.utils")
-    putils.unary_from_softmax = lambda sm, scale=None, clip=1e-5: (-np.log(np.clip(sm, clip, 1.0))).reshape([sm.shape[0], -1]).astype(np.float32)
-    putils.compute_unary = None
-    pkg = types.ModuleType("pydensecrf")
-    pkg.__path__ = []
-    pkg.densecrf, pkg.utils = dcrf, putils
-    sys.modules.update({"pydensecrf": pkg, "pydensecrf.densecrf": dcrf, "pydensecrf.utils": putils})
-    path = os.path.join(refload.REF_ROOT, "manga_translator", "mask_refinement")
-    spec = importlib.util.spec_from_file_location("manga_translator.mask_refinement", os.path.join(path, "__init__.py"), submodule_search_locations=[path])
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules["manga_translator.mask_refinement"] = mod
-    spec.loader.exec_module(mod)
-    return mod
-
-
-@needs_ref
 def test_oracle_dispatch_equals_reference_code_with_restated_dependencies():
     """Pins the statement-order restatement (oracle/mask_refine_ref.py: dispatch, complete_mask, assignment, rectangle arithmetic incl. the
     int32 wrap of empty lines, dilation sizes) on the reference's OWN mask_refinement code, executed unmodified with shapely / pydensecrf
     bound to the oracle's restatements of those two libraries (which remain unpinned themselves)."""
-    import asyncio
-    import warnings
-    warnings.filterwarnings("ignore")
-    ref = _load_reference_mask_refinement()
-    U = refload.load()["utils"]
-    for seed, (h, w, n), offset in ((3, (768, 576, 8), 0), (9, (640, 480, 6), 20)):
-        page, boxes, raw = _page(seed, h, w, n)
-        regions = _regions(boxes) + [types.SimpleNamespace(lines=[np.array([[5.0, 5.0], [60.0, 5.0], [60.0, 30.0], [5.0, 30.0]])])]     # a line without components
-        want = asyncio.run(ref.dispatch(regions, page, raw.copy(), "fit_text", offset, 0, False, 3))
-        got = R.dispatch(regions, page, raw.copy(), U.Quadrilateral, dilation_offset=offset, kernel_size=3)
+    g = _reference()
+    for seed, (h, w, n), offset in cases.REFINE_DISPATCH_CASES:
+        page, regions, raw = cases.refine_dispatch_case(seed, h, w, n)
+        want = g[f"dispatch_{seed}"]
+        got = R.dispatch(regions, page, raw.copy(), geometry.Quadrilateral, dilation_offset=offset, kernel_size=3)
         assert want.dtype == np.uint8 and np.array_equal(got, want), int((got != want).sum())
         assert (want > 0).mean() > 0.02

@@ -1,96 +1,83 @@
-"""Pins the oracle restatement against the unmodified reference modules imported from /root/reference
-(build container only; skipped on the GPU box where the tree is absent)."""
-import warnings
+"""Pins the oracle restatement against the unmodified reference modules.  What the reference computed on these seeded inputs is
+stored under tests/golden/ref_*.{npz,json} (written by oracle/make_reference_golden.py, which runs the reference code), so the
+comparison runs without the reference tree."""
+import json
+import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import cases, nets, refload, weights
+from oracle import cases, nets, weights
 
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not refload.available(), reason="/root/reference not present")]
 torch.set_grad_enabled(False)
 
 
 @pytest.fixture(scope="module")
-def ref():
-    warnings.filterwarnings("ignore")
-    return refload.load()
+def ref(golden_dir):
+    def load(name):
+        path = os.path.join(golden_dir, name)
+        if name.endswith(".json"):
+            with open(path) as f:
+                return json.load(f)
+        return np.load(path)
+    return load
 
 
-def _check_keys(module, sd):
-    want = {k: tuple(v.shape) for k, v in module.state_dict().items()
-            if "num_batches_tracked" not in k and not k.endswith("pe.pe")}
-    have = {k: tuple(v.shape) for k, v in sd.items()}
-    assert want == have
+def _check_keys(spec, sd):
+    have = {k: list(v.shape) for k, v in sd.items()}
+    assert spec == have
 
 
 def test_state_dict_specs_match_reference(ref):
-    _check_keys(ref["det"].DBNetConvNext(), weights.dbnet_weights())
-    _check_keys(ref["ocr"].OCR(["x"] * 300, 768), weights.ocr_weights(300))
+    specs = ref("ref_state_dict_specs.json")
+    _check_keys(specs["dbnet"], weights.dbnet_weights())
+    _check_keys(specs["ocr300"], weights.ocr_weights(300))
     for nb in (9, 18):
-        lf = ref["lama"].LamaFourier(build_discriminator=False, use_mpe=nb == 9, large_arch=nb == 18)
-        _check_keys(lf.generator, weights.lama_weights(nb))
-        if nb == 9:
-            _check_keys(lf.mpe, weights.mpe_weights())
-            assert torch.equal(lf.mpe.rel_pos_emb.weight, weights.mpe_weights()["rel_pos_emb.weight"])
+        _check_keys(specs[f"lama{nb}"], weights.lama_weights(nb))
+    _check_keys(specs["mpe"], weights.mpe_weights())
+    assert torch.equal(torch.from_numpy(ref("ref_lama.npz")["rel_pos_emb"]), weights.mpe_weights()["rel_pos_emb.weight"])
 
 
 def test_dbnet_rectangular(ref):
+    from oracle.make_reference_golden import DBNET_SAMPLE_STRIDE
+    g = ref("ref_dbnet_256x512.npz")
     sd = weights.dbnet_weights(seed=2)
-    net = ref["det"].DBNetConvNext().eval()
-    net.load_state_dict(sd)
     _, x = cases.dbnet_case(256, 512, seed=21)
-    r_db, r_mask = net(x)
     o_db, o_mask = nets.dbnet_forward(sd, x)
-    assert (r_db - o_db).abs().max() < 1e-4 and (r_mask - o_mask).abs().max() < 1e-5
+    o_db = o_db.numpy().reshape(-1)[::DBNET_SAMPLE_STRIDE]
+    assert np.abs(g["db_sample"] - o_db).max() < 1e-4 and np.abs(g["mask"] - o_mask.numpy()).max() < 1e-5
 
 
 def test_ocr_widths_and_decode(ref):
+    g = ref("ref_ocr_widths.npz")
     V = 300
     sd = weights.ocr_weights(V, seed=3)
-    ocr = ref["ocr"].OCR(weights.synthetic_dictionary(V), 768).eval()
-    ocr.load_state_dict(sd, strict=False)
     for wp in (143, 200, 331):
         _, x = cases.ocr_case(3, wp, seed=wp)
-        rl, rc = ocr(x)
+        rl, rc = torch.from_numpy(g[f"logits_{wp}"]), torch.from_numpy(g[f"colors_{wp}"])
         ol, oc = nets.ocr_forward(sd, x)
         assert (rl - ol).abs().max() < 1e-4 and (rc - oc).abs().max() < 1e-5
         idx, lp, col = nets.ocr_top1(sd, x)
-        ref_dec = ocr.decode(x, [0] * 3, 0)
+        ref_dec = [[int(c) for c in row if c >= 0] for row in g[f"decoded_{wp}"]]
         mine = nets.ctc_greedy(idx.numpy(), lp.numpy(), col.numpy())
         top2 = rl.topk(2, dim=-1).values
         if (top2[..., 0] - top2[..., 1]).min() > 1e-3:
-            assert [[int(c[0]) for c in l] for l in ref_dec] == [[c[0] for c in l] for l in mine]
+            assert ref_dec == [[c[0] for c in l] for l in mine]
 
 
 def test_lama_mpe_tables_random_masks(ref):
-    lf = ref["lama"].LamaFourier(build_discriminator=False, use_mpe=True)
-    rng = np.random.default_rng(5)
-    for (h, w) in ((256, 256), (200, 312), (64, 48)):
-        m = np.zeros((h, w), np.float32)
-        for _ in range(4):
-            y, x = rng.integers(0, h - 8), rng.integers(0, w - 8)
-            m[y:y + rng.integers(4, h // 2), x:x + rng.integers(4, w // 2)] = 1
-        rel, _, direct = lf.load_masked_position_encoding(m)
+    g = ref("ref_lama.npz")
+    # random rectangles, then the all-hole and no-hole masks (the reference guards the infinite loop, :778)
+    for i, m in enumerate(cases.mpe_masks()):
         orel, odirect = nets.mpe_tables(m)
-        assert np.array_equal(rel, orel) and np.array_equal(direct, odirect)
-    # all-hole and no-hole masks terminate (the reference guards the infinite loop, :778)
-    for m in (np.zeros((64, 64), np.float32), np.ones((64, 64), np.float32)):
-        rel, _, direct = lf.load_masked_position_encoding(m)
-        orel, odirect = nets.mpe_tables(m)
-        assert np.array_equal(rel, orel) and np.array_equal(direct, odirect)
+        assert np.array_equal(g[f"rel_{i}"], orel) and np.array_equal(g[f"direct_{i}"], odirect)
 
 
 def test_lama_odd_spectrum_sizes(ref):
     sd, msd = weights.lama_weights(9, seed=4), weights.mpe_weights(seed=4)
-    lf = ref["lama"].LamaFourier(build_discriminator=False, use_mpe=True)
-    lf.generator.load_state_dict(sd)
-    lf.mpe.load_state_dict(msd)
-    lf.eval()
     img, mask = cases.lama_case(88, 120, seed=41)   # bottleneck 11x15: odd FFT lengths
-    r = lf(img.clone(), mask)
+    r = torch.from_numpy(ref("ref_lama.npz")["odd_88x120"])
     rel, direct = nets.mpe_tables(mask[0, 0].numpy())
     o = nets.lama_forward(sd, msd, img, mask, torch.from_numpy(rel)[None], torch.from_numpy(direct)[None])
     assert (r - o).abs().max() < 2e-5
@@ -98,125 +85,51 @@ def test_lama_odd_spectrum_sizes(ref):
 
 # ---------------------------------------------------------------------------------------------------------------------
 # The three `_infer` glue paths: oracle/pipeline_ref.py (what the GPU plugin tests compare the product with) against the reference's own
-# `_infer` methods, executed unmodified on the CPU with a duck-typed `self` (constructing the plugin classes would need model
-# directories) and the absent third-party libraries bound to the repo's restatements (pyclipper -> Clipper 6.4.2 restatement, shapely ->
-# geometry restatements).  Closes the loop: reference `_infer` == pipeline_ref here, plugin == pipeline_ref on the GPU.
-def _bind_third_party(ref):
-    import importlib
-    import sys
-    from mit_b200.host import det_post, geometry
-    G = importlib.import_module("manga_translator.utils.generic")
-    du = importlib.import_module("manga_translator.detection.default_utils.dbnet_utils")
-
-    class _Offset:
-        def AddPath(self, box, jt, et):
-            self.box = box
-
-        def Execute(self, d):
-            return [det_post.clipper_offset_round(self.box, d)]
-
-    class Polygon:
-        def __init__(self, pts):
-            self.p = np.asarray(pts, dtype=np.float64).reshape(-1, 2)
-            self.area, self.length = geometry.polygon_area(self.p), geometry.polygon_perimeter(self.p)
-
-        @property
-        def convex_hull(self):
-            return Polygon(geometry._hull(self.p))
-
-        def distance(self, other):
-            return geometry.polygon_distance(self.p, other.p)
-
-    saved = (du.pyclipper, du.Polygon, G.Polygon, G.MultiPoint)
-    du.pyclipper = type("pc", (), dict(PyclipperOffset=_Offset, JT_ROUND=1, ET_CLOSEDPOLYGON=2))
-    du.Polygon = G.Polygon = G.MultiPoint = Polygon
-
-    def restore():
-        du.pyclipper, du.Polygon, G.Polygon, G.MultiPoint = saved
-    return restore
-
-
+# `_infer` methods, executed unmodified on the CPU with a duck-typed `self` and the absent third-party libraries bound to the repo's
+# restatements (pyclipper -> Clipper 6.4.2 restatement, shapely -> geometry restatements).  Closes the loop: reference `_infer` ==
+# pipeline_ref here, plugin == pipeline_ref on the GPU.
 def test_detector_infer_glue_equals_reference_code(ref):
-    import asyncio
-    import logging
-    import types
     from mit_b200 import synth
     from oracle import pipeline_ref
-    det = ref["det"]
+    g = ref("ref_infer_glue.npz")
     sd = {k: v.clone() for k, v in weights.dbnet_weights().items()}
     sd["conv_db.binarize.4.bias"] -= 1.0
-    net = det.DBNetConvNext().eval()
-    net.load_state_dict(sd)
-    det.MODEL = net
-    me = types.SimpleNamespace(device="cpu", logger=logging.getLogger("ref-det"), model=net)
-    restore = _bind_third_party(ref)
-    try:
-        for page, detect_size in ((synth.make_page(5, 512, 384, 6)[0], 512), (synth.make_page(4, 384, 384, 5)[0], 512)):   # pad path; upscale path
-            r_lines, r_mask, _ = asyncio.run(det.DBConvNextDetector._infer(me, page, detect_size, 0.5, 0.6, 2.3))
-            o_lines, o_mask, _, _ = pipeline_ref.detector_infer(sd, page, detect_size, 0.5, 0.6, 2.3)
-            assert len(r_lines) == len(o_lines) and len(r_lines) > 3
-            for a, b in zip(r_lines, o_lines):
-                assert np.array_equal(a.pts, b.pts) and a.prob == b.prob and a.direction == b.direction
-            assert r_mask.dtype == np.uint8 and np.array_equal(r_mask, o_mask)
-    finally:
-        restore()
+    for k, (page, detect_size) in enumerate(((synth.make_page(5, 512, 384, 6)[0], 512), (synth.make_page(4, 384, 384, 5)[0], 512))):   # pad path; upscale path
+        o_lines, o_mask, _, _ = pipeline_ref.detector_infer(sd, page, detect_size, 0.5, 0.6, 2.3)
+        r_pts, r_prob, r_dir, r_mask = g[f"det{k}_pts"], g[f"det{k}_prob"], g[f"det{k}_direction"], g[f"det{k}_mask"]
+        assert len(r_pts) == len(o_lines) and len(r_pts) > 3
+        for pts, prob, d, b in zip(r_pts, r_prob, r_dir, o_lines):
+            assert np.array_equal(pts, b.pts) and prob == b.prob and d == b.direction
+        # the stored mask and this one come from two fp32 CPU evaluations of the network (possibly on different CPUs): the x*255
+        # truncation may flip a pixel by one where the value sits on a boundary, as in the inpainter glue below
+        d = np.abs(r_mask.astype(int) - o_mask.astype(int))
+        assert r_mask.dtype == o_mask.dtype == np.uint8 and d.max() <= 1 and (d > 0).mean() < 1e-3, (int(d.max()), float((d > 0).mean()))
 
 
 def test_ocr_infer_glue_equals_reference_code(ref):
-    import asyncio
-    import logging
-    import sys
-    import types
     from mit_b200 import synth
     from mit_b200.host import geometry
     from oracle import pipeline_ref
+    g = ref("ref_infer_glue.npz")
     V = cases.OCR_VOCAB_SMALL
     dictionary = weights.synthetic_dictionary(V)
     sd = weights.ocr_weights(V)
-    model = ref["ocr"].OCR(dictionary, 768).eval()
-    model.load_state_dict(sd, strict=False)
-    common = sys.modules["manga_translator.ocr.common"]
     page, boxes, _ = synth.make_page(3, 512, 384, 6)
-    U = ref["utils"]
-    restore = _bind_third_party(ref)
-    try:
-        me = types.SimpleNamespace(device="cpu", use_gpu=False, logger=logging.getLogger("ref-ocr"), model=model)
-        me._generate_text_direction = lambda bboxes: common.CommonOCR._generate_text_direction(me, bboxes)
-        r_quads = [U.Quadrilateral(b.copy(), "", 1.0) for b in boxes]
-        cfg = types.SimpleNamespace(ignore_bubble=0, prob=0.0)
-        r_out = asyncio.run(ref["ocr"].Model48pxCTCOCR._infer(me, page, r_quads, cfg, False))
-        o_out = pipeline_ref.ocr_infer(sd, dictionary, page, [geometry.Quadrilateral(b.copy(), "", 1.0) for b in boxes], 0.0)
-        assert len(r_out) == len(o_out) >= 4
-        for a, b in zip(r_out, o_out):
-            assert np.array_equal(a.pts, b.pts) and a.text == b.text and len(a.text) > 0
-            assert abs(a.prob - b.prob) < 1e-4 * max(a.prob, 1e-30)            # the two fp32 network evaluations differ by ~1e-5 in log-probability
-            assert (a.fg_r, a.fg_g, a.fg_b, a.bg_r, a.bg_g, a.bg_b) == (b.fg_r, b.fg_g, b.fg_b, b.bg_r, b.bg_g, b.bg_b)
-    finally:
-        restore()
+    o_out = pipeline_ref.ocr_infer(sd, dictionary, page, [geometry.Quadrilateral(b.copy(), "", 1.0) for b in boxes], 0.0)
+    assert len(g["ocr_pts"]) == len(o_out) >= 4
+    for pts, text, prob, colors, b in zip(g["ocr_pts"], g["ocr_text"], g["ocr_prob"], g["ocr_colors"], o_out):
+        assert np.array_equal(pts, b.pts) and str(text) == b.text and len(b.text) > 0
+        assert abs(prob - b.prob) < 1e-4 * max(prob, 1e-30)            # the two fp32 network evaluations differ by ~1e-5 in log-probability
+        assert tuple(int(c) for c in colors) == (b.fg_r, b.fg_g, b.fg_b, b.bg_r, b.bg_g, b.bg_b)
 
 
 def test_inpainter_infer_glue_equals_reference_code(ref):
-    import asyncio
-    import logging
-    import types
-    from mit_b200 import synth
     from oracle import pipeline_ref
-    lama = ref["lama"]
+    g = ref("ref_infer_glue.npz")
     sd, msd = weights.lama_weights(9), weights.mpe_weights()
-    lf = lama.LamaFourier(build_discriminator=False, use_mpe=True)
-    lf.generator.load_state_dict(sd)
-    lf.mpe.load_state_dict(msd)
-    lf.eval()
-    me = types.SimpleNamespace(device="cpu", logger=logging.getLogger("ref-inp"), model=lf)
-    rng = np.random.default_rng(6)
-    page = rng.integers(0, 256, (200, 152, 3), dtype=np.uint8)
-    mask = np.zeros((200, 152), np.uint8)
-    mask[20:50, 10:120] = 255
-    mask[120:180, 60:90] = 255
-    mask[100:104, 5:40] = 130
-    mask[10, 10] = 127                                            # the 127 / 128 threshold quirk (SURVEY I2)
+    page, mask = cases.inpaint_case()                             # incl. the 127 / 128 threshold quirk (SURVEY I2)
     for size in (1024, 128):                                      # no resize; keep-aspect resize + back
-        r = asyncio.run(lama.LamaMPEInpainter._infer(me, page.copy(), mask.copy(), types.SimpleNamespace(inpainting_precision="fp32"), size, False))
+        r = g[f"inpaint_{size}"]
         o, _ = pipeline_ref.lama_infer(sd, msd, page.copy(), mask.copy(), size)
         assert r.dtype == o.dtype == np.uint8 and r.shape == page.shape
         d = np.abs(r.astype(int) - o.astype(int))
@@ -228,14 +141,11 @@ def test_common_detector_detect_equals_reference_code(ref):
     auto-rotation; used when the reference package cannot be imported) against the reference's own `detection/common.py` code, both
     wrapped around the same stub `_detect`: identical text lines, raw mask and mask for every combination of the switches."""
     import asyncio
-    import importlib
-    import itertools
     import importlib.util
     import sys
     from mit_b200 import compat as _compat_loaded
     from mit_b200.host import geometry
-    rc = importlib.import_module("manga_translator.detection.common")
-    # a second copy of mit_b200/compat.py imported while `manga_translator` is hidden: that is the stand-in the GPU box gets
+    # a second copy of mit_b200/compat.py imported while `manga_translator` is hidden: the stand-in, even where the package is installed
     hidden = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "manga_translator" or k.startswith("manga_translator.")}
     sys.modules["manga_translator"] = None                       # makes `import manga_translator...` raise ImportError
     try:
@@ -247,29 +157,9 @@ def test_common_detector_detect_equals_reference_code(ref):
         del sys.modules["manga_translator"]
         sys.modules.update(hidden)
     assert not compat.HAVE_REFERENCE
-    U = ref["utils"]
-    restore = _bind_third_party(ref)
-
-    def stub(quad_cls):
-        async def _detect(self, image, detect_size, text_threshold, box_threshold, unclip_ratio, verbose=False):
-            self.seen.append(image.copy())
-            h, w = image.shape[:2]
-            rng = np.random.default_rng(h * 7919 + w)
-            lines = []
-            for _ in range(6):
-                x0, y0 = int(rng.integers(0, w - 40)), int(rng.integers(0, h - 40))
-                bw, bh = int(rng.integers(12, 120)), int(rng.integers(8, 60))
-                lines.append(quad_cls(np.array([[x0, y0], [x0 + bw, y0], [x0 + bw, y0 + bh], [x0, y0 + bh]]), "", 0.9))
-            lines.append(quad_cls(np.array([[5, 5], [6, 5], [6, 6], [5, 6]]), "", 0.5))          # area 1: filtered
-            raw = (rng.random((h, w)) * 255).astype(np.uint8)
-            return lines, raw, (rng.random((h, w)) > 0.5).astype(np.uint8) * 255
-        return _detect
-
-    class RefDet(rc.CommonDetector):
-        _detect = stub(U.Quadrilateral)
 
     class OurDet(compat.OfflineDetector):
-        _detect = stub(geometry.Quadrilateral)
+        _detect = cases.detect_variant_stub(geometry.Quadrilateral)
 
         async def _load(self, device):
             pass
@@ -280,17 +170,13 @@ def test_common_detector_detect_equals_reference_code(ref):
         async def _infer(self, *a, **k):
             raise AssertionError("not used: `_detect` is stubbed")
 
-    try:
-        rng = np.random.default_rng(2)
-        for (h, w) in ((300, 200), (520, 450), (380, 700)):
-            img = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-            for invert, gamma, rotate, auto in itertools.product((False, True), repeat=4):
-                r, o = RefDet(), OurDet()
-                r.seen, o.seen = [], []
-                rt, rraw, rmask = asyncio.run(r.detect(img.copy(), 1024, 0.5, 0.7, 2.3, invert, gamma, rotate, auto))
-                ot, oraw, omask = asyncio.run(o.detect(img.copy(), 1024, 0.5, 0.7, 2.3, invert, gamma, rotate, auto))
-                assert len(r.seen) == len(o.seen) and all(np.array_equal(a, b) for a, b in zip(r.seen, o.seen)), (h, w, invert, gamma, rotate, auto)
-                assert len(rt) == len(ot) and all(np.array_equal(a.pts, b.pts) for a, b in zip(rt, ot))
-                assert np.array_equal(rraw, oraw) and np.array_equal(rmask, omask)
-    finally:
-        restore()
+    runs = ref("ref_detect_variants.json")["runs"]
+    variants = list(cases.detect_variant_cases())
+    assert len(runs) == len(variants) == 48
+    for want, (img, invert, gamma, rotate, auto) in zip(runs, variants):
+        o = OurDet()
+        o.seen = []
+        ot, oraw, omask = asyncio.run(o.detect(img.copy(), 1024, 0.5, 0.7, 2.3, invert, gamma, rotate, auto))
+        assert want["seen"] == [cases.digest(a) for a in o.seen], (img.shape, invert, gamma, rotate, auto)
+        assert want["lines"] == [np.asarray(t.pts).tolist() for t in ot]
+        assert want["raw"] == cases.digest(oraw) and want["mask"] == cases.digest(omask)

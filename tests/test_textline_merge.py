@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-from mit_b200.host import textline_merge
+from mit_b200.host import geometry, textline_merge
 from mit_b200.host.geometry import Quadrilateral
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "textline_merge.json")
@@ -117,133 +117,54 @@ def test_pair_matrix_glue_with_a_fake_engine():
     assert [d for _, d in geometry.generate_text_direction(quads, engine=fake)] == [d for _, d in geometry.generate_text_direction(quads)]
 
 
+REFERENCE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_textline_merge.json")
+
+
 def test_merge_predicate_equals_reference_code():
-    """`host.geometry.can_merge_region` against the reference's own `quadrilateral_can_merge_region` (utils/generic.py:653-698), executed
-    unmodified with shapely's Polygon bound to our polygon-distance restatement: every pair of every known-answer case and of a set of
-    rotated random quads, under both parameter sets in use.  Pins the rule cascade and its numpy scalar-type semantics (the distance
-    function itself is the restated part)."""
+    """`host.geometry.can_merge_region` against the reference's own `quadrilateral_can_merge_region` (utils/generic.py:653-698), run
+    unmodified with shapely's Polygon bound to our polygon-distance restatement (its verdicts are stored in tests/golden): every pair of
+    every known-answer case and of a set of rotated random quads, under both parameter sets in use.  Pins the rule cascade and its numpy
+    scalar-type semantics (the distance function itself is the restated part)."""
     import itertools
-    from oracle import refload
-    if not refload.available():
-        pytest.skip("/root/reference not present")
-    import warnings
-    warnings.filterwarnings("ignore")
-    from mit_b200.host import geometry
-    U = refload.load()["utils"]
-    G = __import__("manga_translator.utils.generic", fromlist=["x"])
-
-    class Polygon:
-        def __init__(self, pts):
-            self.p = np.asarray(pts, dtype=np.float64).reshape(-1, 2)
-
-        def distance(self, other):
-            return geometry.polygon_distance(self.p, other.p)
-
-    saved = G.Polygon
-    G.Polygon = Polygon
-    try:
-        rng = np.random.default_rng(8)
-        sets = [[np.array(l) for l in c["lines"]] for c in CASES]
-        rnd = []
-        for t in range(60):
-            cx, cy = rng.uniform(200, 500), rng.uniform(200, 500)
-            ww, hh = rng.uniform(30, 200), rng.uniform(12, 40)
-            if t % 3 == 0:
-                ww, hh = hh, ww
-            ang = rng.uniform(-0.5, 0.5) if t % 2 else 0.0
-            c, s = np.cos(ang), np.sin(ang)
-            rnd.append((np.array([[-ww / 2, -hh / 2], [ww / 2, -hh / 2], [ww / 2, hh / 2], [-ww / 2, hh / 2]]) @ np.array([[c, s], [-s, c]]) + [cx, cy]).astype(np.int64))
-        sets.append(rnd)
-        n_true = n_pairs = 0
-        for pts_list in sets:
-            mine = [Quadrilateral(p, "", 1.0) for p in pts_list]
-            ref = [U.Quadrilateral(p, "", 1.0) for p in pts_list]
-            for r, m in zip(ref, mine):                       # the angled branch asks Quadrilateral.poly_distance (hull polygons)
-                r.__dict__["polygon"] = Polygon(geometry._hull(m.pts))
-            for params in (dict(aspect_ratio_tol=1), dict(aspect_ratio_tol=1.3, font_size_ratio_tol=2, char_gap_tolerance=1, char_gap_tolerance2=3)):
-                for u, v in itertools.combinations(range(len(mine)), 2):
-                    want = bool(G.quadrilateral_can_merge_region(ref[u], ref[v], **params))
-                    assert bool(geometry.can_merge_region(mine[u], mine[v], **params)) == want, (u, v, params)
-                    n_true += want
-                    n_pairs += 1
-        assert n_true > 50 and n_pairs > 3000
-    finally:
-        G.Polygon = saved
+    from oracle import cases
+    with open(REFERENCE) as f:
+        want_sets = json.load(f)["predicate"]
+    sets = [[np.array(l) for l in c["lines"]] for c in CASES] + [cases.merge_random_quads()]
+    assert len(sets) == len(want_sets)
+    n_true = n_pairs = 0
+    for pts_list, want_per_params in zip(sets, want_sets):
+        mine = [Quadrilateral(p, "", 1.0) for p in pts_list]
+        for params, want in zip(cases.MERGE_PARAMS, want_per_params):
+            got = "".join("1" if geometry.can_merge_region(mine[u], mine[v], **params) else "0"
+                          for u, v in itertools.combinations(range(len(mine)), 2))
+            assert got == want, params
+            n_true += want.count("1")
+            n_pairs += len(want)
+    assert n_true > 50 and n_pairs > 3000
 
 
 def test_regions_and_direction_graph_equal_reference_code_on_random_pages():
     """Beyond the 11 known-answer cases: the reference's own `merge_bboxes_text_region` (textline_merge/__init__.py:110-181) and
-    `CommonOCR._generate_text_direction` (ocr/common.py:12-39), executed unmodified with shapely bound to our geometry restatements, against
-    `host.textline_merge.merge_text_regions` / `host.geometry.generate_text_direction` on random clustered pages of rotated lines."""
-    import importlib.util
-    import sys
-    from oracle import refload
-    if not refload.available():
-        pytest.skip("/root/reference not present")
-    import warnings
-    warnings.filterwarnings("ignore")
-    from mit_b200.host import geometry
-    U = refload.load()["utils"]
-    G = __import__("manga_translator.utils.generic", fromlist=["x"])
-    common = sys.modules["manga_translator.ocr.common"]
-
-    class Polygon:
-        def __init__(self, pts):
-            self.p = np.asarray(pts, dtype=np.float64).reshape(-1, 2)
-
-        @property
-        def area(self):
-            return geometry.polygon_area(self.p)
-
-        @property
-        def convex_hull(self):
-            return Polygon(geometry._hull(self.p))
-
-        def distance(self, other):
-            return geometry.polygon_distance(self.p, other.p)
-
-    class MultiPoint(Polygon):
-        pass
-
-    path = os.path.join(refload.REF_ROOT, "manga_translator", "textline_merge", "__init__.py")
-    spec = importlib.util.spec_from_file_location("manga_translator.textline_merge", path, submodule_search_locations=[os.path.dirname(path)])
-    ref_merge = importlib.util.module_from_spec(spec)
-    sys.modules["manga_translator.textline_merge"] = ref_merge
-    spec.loader.exec_module(ref_merge)
-    saved = (G.Polygon, G.MultiPoint, ref_merge.Polygon)
-    G.Polygon, G.MultiPoint, ref_merge.Polygon = Polygon, MultiPoint, Polygon
-    try:
-        rng = np.random.default_rng(21)
-        n_regions = 0
-        for page in range(12):
-            pts_list = []
-            for blk in range(int(rng.integers(2, 5))):           # a few "speech bubbles" of stacked lines + stray lines
-                bx, by = rng.uniform(100, 900), rng.uniform(100, 700)
-                vertical = rng.random() < 0.5
-                fs = rng.uniform(18, 40)
-                ang = rng.uniform(-0.12, 0.12) if rng.random() < 0.4 else 0.0
-                for k in range(int(rng.integers(1, 6))):
-                    ln = rng.uniform(60, 260)
-                    w, h = (fs, ln) if vertical else (ln, fs)
-                    cx, cy = (bx - k * fs * rng.uniform(1.05, 1.6), by + rng.uniform(-8, 8)) if vertical else (bx + rng.uniform(-8, 8), by + k * fs * rng.uniform(1.05, 1.6))
-                    c, s = np.cos(ang), np.sin(ang)
-                    pts_list.append((np.array([[-w / 2, -h / 2], [w / 2, -h / 2], [w / 2, h / 2], [-w / 2, h / 2]]) @ np.array([[c, s], [-s, c]]) + [cx, cy]).astype(np.int64))
-            cols = [tuple(int(v) for v in rng.integers(0, 256, 6)) for _ in pts_list]
-            mine = [Quadrilateral(p, f"t{i}", 0.9, *c) for i, (p, c) in enumerate(zip(pts_list, cols))]
-            ref = [U.Quadrilateral(p, f"t{i}", 0.9, *c) for i, (p, c) in enumerate(zip(pts_list, cols))]
-            for q in mine + ref:
-                q.assigned_direction = q.direction
-            want = [([ref.index(q) for q in tl], fg, bg) for tl, fg, bg in ref_merge.merge_bboxes_text_region(ref, 1000, 800)]
-            got = [(list(members), fg, bg) for members, fg, bg, _ in textline_merge.merge_text_regions(mine, 1000, 800)]
-            key = lambda r: tuple(sorted(r[0]))
-            assert sorted(map(key, got)) == sorted(map(key, want))                                       # same partition ...
-            assert sorted(got, key=key) == sorted(want, key=key), (page, got, want)                      # ... same reading order and colours
-            n_regions += len(want)
-            rd = [(ref.index(q), d) for q, d in common.CommonOCR._generate_text_direction(None, ref)]
-            md = [(mine.index(q), d) for q, d in geometry.generate_text_direction(mine)]
-            assert sorted(rd) == sorted(md)
-            # the order of whole groups follows networkx's component iteration in both; within a group it must agree
-            assert rd == md, (page, rd, md)
-        assert n_regions > 30
-    finally:
-        G.Polygon, G.MultiPoint, ref_merge.Polygon = saved
+    `CommonOCR._generate_text_direction` (ocr/common.py:12-39), run unmodified with shapely bound to our geometry restatements (their
+    results are stored in tests/golden), against `host.textline_merge.merge_text_regions` / `host.geometry.generate_text_direction` on
+    random clustered pages of rotated lines."""
+    from oracle import cases
+    with open(REFERENCE) as f:
+        want_pages = json.load(f)["pages"]
+    n_regions = 0
+    for page, ((pts_list, cols), ref) in enumerate(zip(cases.merge_random_pages(), want_pages)):
+        mine = [Quadrilateral(p, f"t{i}", 0.9, *c) for i, (p, c) in enumerate(zip(pts_list, cols))]
+        for q in mine:
+            q.assigned_direction = q.direction
+        want = [(members, tuple(fg), tuple(bg)) for members, fg, bg in ref["regions"]]
+        got = [(list(members), tuple(int(v) for v in fg), tuple(int(v) for v in bg)) for members, fg, bg, _ in textline_merge.merge_text_regions(mine, 1000, 800)]
+        key = lambda r: tuple(sorted(r[0]))
+        assert sorted(map(key, got)) == sorted(map(key, want))                                       # same partition ...
+        assert sorted(got, key=key) == sorted(want, key=key), (page, got, want)                      # ... same reading order and colours
+        n_regions += len(want)
+        rd = [tuple(x) for x in ref["directions"]]
+        md = [(mine.index(q), d) for q, d in geometry.generate_text_direction(mine)]
+        assert sorted(rd) == sorted(md)
+        # the order of whole groups follows networkx's component iteration in both; within a group it must agree
+        assert rd == md, (page, rd, md)
+    assert len(want_pages) == 12 and n_regions > 30
