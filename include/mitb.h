@@ -131,7 +131,9 @@ int mitb_op_irfft2(mitb_ctx* ctx, const float* spec, int c, int h, int w, float*
  * irfft adds `add` [n,h,w,c] when non-NULL (the x + fu(x) residual, inpainting_lama_mpe.py:305).  h, w {2,3,5}-smooth, c even. */
 int mitb_op_rfft2_nhwc(mitb_ctx* ctx, const float* x, int n, int h, int w, int c, float* spec, void* stream);
 int mitb_op_irfft2_nhwc(mitb_ctx* ctx, const float* spec, const float* add, int n, int h, int w, int c, float* y, void* stream);
-/* Multi-head attention core: qk [n*t, 2*d] (q then k, already projected), v [n*t, d] -> out [n*t, d]. */
+/* Multi-head attention core: qk [n*t, 2*d] (q then k, already projected), v [n*t, d] -> out [n*t, d], d = heads * head_dim, no mask.
+ * Any alignment.  Any t for head_dim <= 64 (the OCR: 8 x 40, t <= 2048); for head_dim > 64 only t with
+ * 4 * (2 * t * (head_dim + 1) + 8 * t + 8 * head_dim) <= 200 KB (K / V of a head held whole in shared memory), else an error. */
 int mitb_op_attention(mitb_ctx* ctx, const float* qk, const float* v, int n, int t, int heads, int head_dim,
                       float* out, void* stream);
 /* LamaFourier.load_masked_position_encoding at its 256x256 working resolution (inpainting_lama_mpe.py:763-803): small = the

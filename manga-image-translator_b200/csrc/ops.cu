@@ -491,6 +491,97 @@ __global__ void __launch_bounds__(256) attention40_kernel(const float* __restric
   }
 }
 
+// Sequences whose whole K / V does not fit in shared memory (the OCR reads lines up to T = 2048, the rows of its positional-encoding
+// table): K / V of the head stream through shared memory in chunks of AS_TK keys under an online softmax.  Per query row a running max
+// m and sum l; when a chunk raises the max, l and the output accumulators are rescaled by exp(m_old - m_new).  Each warp owns AS_R
+// consecutive query rows (a CTA covers nw * AS_R rows and streams K / V once for all of them); lane j scores key j of each 32-key group,
+// output dimension d lives in lane d % 32, register d / 32.  4-byte loads only, so any alignment; head_dim <= 32 * AS_HDR.
+constexpr int AS_TK = 64, AS_R = 4, AS_HDR = 2;
+__global__ void __launch_bounds__(256) attention_stream_kernel(const float* __restrict__ qk, const float* __restrict__ v, float* __restrict__ out,
+                                                               int T, int heads, int hd, float scale) {
+  extern __shared__ float sm[];
+  const int D = heads * hd, ld = hd + 1;
+  const int n = blockIdx.x / heads, h = blockIdx.x % heads;
+  const int nw = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float* Ks = sm; float* Vs = Ks + AS_TK * ld;
+  float* Q = Vs + AS_TK * ld + (size_t)warp * AS_R * hd;   // [nw][AS_R][hd]
+  const int row0 = (blockIdx.y * nw + warp) * AS_R;
+  for (int i = lane; i < AS_R * hd; i += 32) {
+    const int t = row0 + i / hd;
+    Q[i] = t < T ? qk[((size_t)n * T + t) * 2 * D + h * hd + i % hd] : 0.f;
+  }
+  float m[AS_R], l[AS_R], acc[AS_R][AS_HDR];
+#pragma unroll
+  for (int r = 0; r < AS_R; ++r) {
+    m[r] = -INFINITY; l[r] = 0.f;
+#pragma unroll
+    for (int i = 0; i < AS_HDR; ++i) acc[r][i] = 0.f;
+  }
+  for (int k0 = 0; k0 < T; k0 += AS_TK) {
+    const int nk = min(AS_TK, T - k0);
+    __syncthreads();                                           // the previous chunk is consumed (and, the first time, Q is staged)
+    for (int i = threadIdx.x; i < nk * hd; i += blockDim.x) {
+      const int j = i / hd, d = i % hd;
+      const size_t row = (size_t)n * T + k0 + j;
+      Ks[j * ld + d] = qk[row * 2 * D + D + h * hd + d];
+      Vs[j * ld + d] = v[row * D + h * hd + d];
+    }
+    __syncthreads();
+    for (int j0 = 0; j0 < nk; j0 += 32) {
+      const int j = j0 + lane;
+      float s[AS_R];
+#pragma unroll
+      for (int r = 0; r < AS_R; ++r) s[r] = 0.f;
+      if (j < nk) {
+        for (int d = 0; d < hd; ++d) {
+          const float kd = Ks[j * ld + d];
+#pragma unroll
+          for (int r = 0; r < AS_R; ++r) s[r] = fmaf(Q[r * hd + d], kd, s[r]);
+        }
+      }
+#pragma unroll
+      for (int r = 0; r < AS_R; ++r) {
+        const float sr = j < nk ? s[r] * scale : -INFINITY;
+        float cm = sr;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) cm = fmaxf(cm, __shfl_xor_sync(0xffffffffu, cm, o));
+        const float mn = fmaxf(m[r], cm);                      // finite: lane 0 always holds a key of this group
+        const float c = expf(m[r] - mn);                       // 0 on the first group (m = -inf)
+        s[r] = expf(sr - mn);                                  // 0 for the lanes past the last key
+        l[r] = fmaf(l[r], c, s[r]);                            // per-lane partial sum, reduced at the end
+#pragma unroll
+        for (int i = 0; i < AS_HDR; ++i) acc[r][i] *= c;
+        m[r] = mn;
+      }
+      const int kn = min(32, nk - j0);
+      for (int jj = 0; jj < kn; ++jj) {
+        const float* vr = Vs + (j0 + jj) * ld;
+        float vd[AS_HDR];
+#pragma unroll
+        for (int i = 0; i < AS_HDR; ++i) vd[i] = lane + 32 * i < hd ? vr[lane + 32 * i] : 0.f;
+#pragma unroll
+        for (int r = 0; r < AS_R; ++r) {
+          const float p = __shfl_sync(0xffffffffu, s[r], jj);
+#pragma unroll
+          for (int i = 0; i < AS_HDR; ++i) acc[r][i] = fmaf(p, vd[i], acc[r][i]);
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < AS_R; ++r) {
+    float sum = l[r];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+    const int t = row0 + r;
+    if (t >= T) continue;
+    const float inv = 1.f / sum;
+#pragma unroll
+    for (int i = 0; i < AS_HDR; ++i)
+      if (lane + 32 * i < hd) out[((size_t)n * T + t) * D + h * hd + lane + 32 * i] = acc[r][i] * inv;
+  }
+}
+
 void launch_attention(const float* qk, const float* v, float* out, int N, int T, int heads, int hd, cudaStream_t st) {
   if (hd == AT_HD && (((uintptr_t)qk | (uintptr_t)v) & 15) == 0) {
     const int threads = 256, nw = threads / 32;
@@ -507,7 +598,18 @@ void launch_attention(const float* qk, const float* v, float* out, int N, int T,
   }
   const int threads = 256;
   const size_t smem = ((size_t)2 * T * (hd + 1) + (size_t)(threads / 32) * T + (size_t)(threads / 32) * hd) * sizeof(float);
-  MITB_CHECK(smem <= 200 * 1024, "attention: sequence too long (T=%d)", T);
+  if (smem > 200 * 1024) {
+    MITB_CHECK(hd <= 32 * AS_HDR, "attention: sequence too long (T=%d) for head_dim %d; longer sequences need head_dim <= %d", T, hd,
+               32 * AS_HDR);
+    const int nw = threads / 32, rows = nw * AS_R;
+    MITB_CHECK(N >= 1 && heads >= 1 && (long)N * heads <= INT_MAX && (T + rows - 1) / rows <= 65535, "attention: bad shape n=%d t=%d heads=%d",
+               N, T, heads);
+    const size_t ssm = ((size_t)2 * AS_TK * (hd + 1) + (size_t)rows * hd) * sizeof(float);   // <= 41.5 KB: no opt-in needed
+    ProfScope ps("attention", 4.0 * N * heads * (double)T * T * hd, 16.0 * N * T * heads * hd, st);
+    attention_stream_kernel<<<dim3(N * heads, (T + rows - 1) / rows), threads, ssm, st>>>(qk, v, out, T, heads, hd, 1.0f / sqrtf((float)hd));
+    LAUNCH_END();
+    return;
+  }
   static PerDeviceOnce attr_set;
   if (attr_set.first()) CUDA_OK(cudaFuncSetAttribute(attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   ProfScope ps("attention", 4.0 * N * heads * (double)T * T * hd, 16.0 * N * T * heads * hd, st);

@@ -4,7 +4,7 @@ The tests that pin the oracle and the host ports on the reference's own code com
 without the reference tree.  Where the reference code calls a third-party library that is not installed (pyclipper, shapely,
 pydensecrf), it runs with that library bound to the repository's restatement, exactly as the tests did when they ran it live.
 
-  python -m oracle.make_reference_golden
+  python -m oracle.make_reference_golden [section ...]     (default: every section; e.g. `ocr_long` writes ref_ocr_long.npz only)
 
 Large arrays that must match exactly are stored as oracle.cases.digest() values; one dense output is stored as a strided
 sample.  No file is larger than 1 MB.
@@ -200,6 +200,37 @@ def networks(ref):
     _save_npz("ref_lama.npz", **out)
 
 
+OCR_LONG_WIDTHS = (2439, 8196)   # T = 608 (a caption across a 1536 px page, 32 px tall) and T = 2048, the positional table's length
+OCR_LONG_TOO_WIDE = 8200         # T = 2049
+
+
+def ocr_long(ref):
+    """The reference OCR on two-line chunks of the longest lines it reads.  Compact per-step results instead of the logits (at T = 2048
+    those alone are 2.4 MB): argmax, max log-softmax, top-2 logit margin, clamped colours, and the decoded character ids."""
+    V = 300
+    ocr = ref["ocr"].OCR(weights.synthetic_dictionary(V), 768).eval()
+    ocr.load_state_dict(weights.ocr_weights(V, seed=3), strict=False)
+    out = {}
+    for wp in OCR_LONG_WIDTHS:
+        _, x = cases.ocr_case(2, wp, seed=wp)
+        rl, rc = ocr(x)
+        lp, idx = rl.log_softmax(2).max(2)
+        top2 = rl.topk(2, dim=-1).values
+        dec = ocr.decode(x, [0] * 2, 0)
+        chars = np.full((2, max(1, max(len(l) for l in dec))), -1, np.int16)
+        for i, l in enumerate(dec):
+            chars[i, :len(l)] = [int(c[0]) for c in l]
+        out.update({f"argmax_{wp}": idx.numpy().astype(np.int16), f"logprob_{wp}": lp.numpy(),
+                    f"margin_{wp}": (top2[..., 0] - top2[..., 1]).numpy(), f"colors_{wp}": rc.clamp(0, 1).numpy(), f"decoded_{wp}": chars})
+    _, x = cases.ocr_case(2, OCR_LONG_TOO_WIDE, seed=OCR_LONG_TOO_WIDE)
+    try:
+        ocr(x)
+        out["too_wide_raises"] = np.array(False)
+    except RuntimeError:                          # x + pe[:, :T] with T = 2049 against a 2048-row table: a shape mismatch
+        out["too_wide_raises"] = np.array(True)
+    _save_npz("ref_ocr_long.npz", **out)
+
+
 # ------------------------------------------------------------------------------------------------ the three `_infer` glue paths
 def infer_glue(ref):
     from mit_b200 import synth
@@ -380,22 +411,25 @@ def textline_merge(ref):
     _save_json("ref_textline_merge.json", doc)
 
 
-def main():
+SECTIONS = {f.__name__: f for f in (networks, ocr_long, infer_glue, detect_variants, host, mask_refinement, textline_merge)}
+
+
+def main(sections=None):
+    sections = sections or list(SECTIONS)
+    unknown = [s for s in sections if s not in SECTIONS]
+    if unknown:
+        raise SystemExit(f"unknown section(s) {unknown}; choose from {list(SECTIONS)}")
     warnings.filterwarnings("ignore")
     if PKG_ROOT not in sys.path:
         sys.path.insert(0, PKG_ROOT)
     torch.set_grad_enabled(False)
     ref = refload.load()
-    networks(ref)
-    infer_glue(ref)
-    detect_variants(ref)
-    host(ref)
-    mask_refinement(ref)
-    textline_merge(ref)
+    for name in sections:
+        SECTIONS[name](ref)
     for f in sorted(os.listdir(OUT)):
         if f.startswith("ref_"):
             print(f, os.path.getsize(os.path.join(OUT, f)))
 
 
 if __name__ == "__main__":
-    sys.exit(main())
+    sys.exit(main(sys.argv[1:]))

@@ -66,6 +66,31 @@ def test_ocr_widths_and_decode(ref):
             assert ref_dec == [[c[0] for c in l] for l in mine]
 
 
+def test_ocr_long_lines(ref):
+    """The oracle on the longest lines the reference reads: T = 608 and T = 2048 (its PositionalEncoding has 2048 rows, so the oracle's
+    per-call sinusoid_pe(T) is checked against the reference's table at every position), and the reference refuses T = 2049."""
+    from oracle.make_reference_golden import OCR_LONG_TOO_WIDE, OCR_LONG_WIDTHS
+    g = ref("ref_ocr_long.npz")
+    sd = weights.ocr_weights(300, seed=3)
+    for wp in OCR_LONG_WIDTHS:
+        _, x = cases.ocr_case(2, wp, seed=wp)
+        logits, colors = nets.ocr_forward(sd, x)
+        assert logits.shape[1] == (wp // 2) // 2 - 1
+        lp, idx = logits.log_softmax(2).max(2)
+        top2 = logits.topk(2, dim=-1).values
+        safe = g[f"margin_{wp}"] > 1e-3
+        assert safe.mean() > 0.99
+        assert np.array_equal(idx.numpy()[safe], g[f"argmax_{wp}"][safe])
+        assert np.abs(lp.numpy() - g[f"logprob_{wp}"]).max() < 1e-4
+        assert np.abs((top2[..., 0] - top2[..., 1]).numpy() - g[f"margin_{wp}"]).max() < 2e-4
+        assert np.abs(colors.clamp(0, 1).numpy() - g[f"colors_{wp}"]).max() < 1e-5
+        # decode: the oracle's argmax on the safe steps, the reference's on the few near-ties
+        mixed = np.where(safe, idx.numpy(), g[f"argmax_{wp}"])
+        mine = nets.ctc_greedy(mixed, lp.numpy(), colors.clamp(0, 1).numpy())
+        assert [[int(c) for c in row if c >= 0] for row in g[f"decoded_{wp}"]] == [[c[0] for c in l] for l in mine]
+    assert (OCR_LONG_TOO_WIDE // 2) // 2 - 1 == 2049 and bool(g["too_wide_raises"])
+
+
 def test_lama_mpe_tables_random_masks(ref):
     g = ref("ref_lama.npz")
     # random rectangles, then the all-hole and no-hole masks (the reference guards the infinite loop, :778)

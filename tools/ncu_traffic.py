@@ -23,7 +23,7 @@ CLASSES = (  # first match wins; conv_tc = every kernel a dense conv op launches
     ("fft", ("rfft_rows", "irfft_rows", "fft_cols")),
     ("dwconv7_ln", ("dwconv7_ln_kernel",)),
     ("layernorm", ("layernorm_kernel",)),
-    ("attention", ("attention_kernel", "attention40_kernel")),
+    ("attention", ("attention_kernel", "attention40_kernel", "attention_stream_kernel")),
     ("ocr_crops_ctc", ("warp_lines_kernel", "ctc_collapse_kernel")),
     ("need_maps", ("need_from_mask_kernel", "need_pool2_kernel", "need_dilate1_kernel")),
     ("bilateral", ("bilateral17_kernel",)),
